@@ -169,7 +169,7 @@ def test_thin_layers_fast_mode(ast, cin, cout, k, norm, h, w):
 
 
 @pytest.mark.parametrize("w", [13, 300])          # 300: wider than one 256-column block segment
-def test_fold_rows_matches_direct_sum(w):
+def test_fold_rows_matches_direct_sum(ast, w):
     """ast_fold_rows: out[n,y,x,c] = bias[c] + sum_d part[n,y,x+d,d*C+c] (NCHW output view, optional ReLU)."""
     from artist_style_transfer_b200 import ops
     torch.manual_seed(5)
