@@ -16,7 +16,6 @@ AST_MAX_TAPS = 81
 CONV_RELU, CONV_REFLECT, CONV_TENSOR = 1, 2, 4
 CONV_POOL_ONLY = 16
 CONV_ROUND_TF32 = 8
-IN_SUMS_ZEROED = 2
 GRAM_COUNTERS_PER_IMAGE = 16
 
 _DTYPES = {torch.float32: AST_F32, torch.bfloat16: AST_BF16, torch.uint8: AST_U8, torch.float16: AST_F16}
@@ -87,10 +86,6 @@ _SIGNATURES = {
     "ast_instnorm_stats": [_P(Image), _vp, _vp, ctypes.c_float, _vp, _vp],
     "ast_instnorm_finalize": [_vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_float, _vp, _vp, _vp],
     "ast_instnorm_apply": [_P(Image), _vp, _vp, _vp, _vp, _P(Image), _P(Image), ctypes.c_int32, ctypes.c_int32, _vp],
-    "ast_instnorm_bwd_stats": [_P(Image), _vp, _vp, _vp, _vp, _P(Image), ctypes.c_int32, _P(Image), ctypes.c_int32,
-                               _vp, _vp, _vp],
-    "ast_instnorm_bwd_apply": [_P(Image), _vp, _vp, _vp, _vp, _P(Image), ctypes.c_int32, _P(Image), ctypes.c_int32,
-                               _vp, _vp, _P(Image), _P(Image), _vp],
     "ast_instnorm_bwd": [_P(Image), _vp, _vp, _vp, _vp, _P(Image), ctypes.c_int32, _P(Image), ctypes.c_int32,
                          _vp, _vp, _vp, _P(Image), _P(Image), _vp],
     "ast_maxpool2_fwd": [_P(Image), _P(Image), _P(Image), _vp],

@@ -277,7 +277,7 @@ class _StageFunction(torch.autograd.Function):
                 bank_it -= 1
                 s12 = banks[bank_off[bank_it]:bank_off[bank_it] + 2 * n * c].view(2, n * c)
                 ops.instnorm_bwd(raw, mean, rstd, gam.detach(), bet.detach(), gpad[j], node_pad[j],
-                                 gextra[j], st.relu, d_raw, gtotal, s12=s12, zeroed=True,
+                                 gextra[j], st.relu, d_raw, gtotal, s12=s12,
                                  arrive=arrive_all[bank_it * nb:(bank_it + 1) * nb])
                 if gtotal is not None:
                     assert gextra[st.res_from + 1] is None

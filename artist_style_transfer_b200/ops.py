@@ -270,19 +270,20 @@ def _instnorm_apply_impl(x, mean, rstd, gamma, beta, out, pad, relu, residual=No
     return out
 
 
-def _instnorm_bwd_impl(x, mean, rstd, gamma, beta, gpad, pad, gextra, relu, dx, gtotal=None, s12=None, zeroed=False,
-                       arrive=None):
+def _instnorm_bwd_impl(x, mean, rstd, gamma, beta, gpad, pad, gextra, relu, dx, gtotal=None, s12=None, arrive=None):
     """Returns s12 of shape (2, N*C): dbeta = s12[0].view(N,C).sum(0), dgamma = s12[1].view(N,C).sum(0); fills dx
-    (and gtotal).  `s12` may be a caller-provided (2, N*C) fp32 view (e.g. a slice of one buffer shared by layers)."""
+    (and gtotal).  `s12` may be a caller-provided (2, N*C) fp32 view (e.g. a slice of one buffer shared by layers) and
+    `arrive` N int32 barrier counters; both must be zero-filled.  Zeroed buffers are allocated for those not given."""
     n, _, _, c = x.shape
     if s12 is None:
-        s12 = torch.empty((2, n * c), dtype=torch.float32, device=x.device)  # one allocation: the caller reduces both
+        s12 = torch.zeros((2, n * c), dtype=torch.float32, device=x.device)  # one allocation: the caller reduces both
     s1, s2 = s12[0], s12[1]                                                  # over the batch with one kernel
+    if arrive is None:
+        arrive = torch.zeros(n, dtype=torch.int32, device=x.device)
     lib = _lib.load()
     xi, gp, ge, dxi, gt = image(x), image(gpad), image(gextra), image(dx), image(gtotal)
-    flags = int(relu) | (_lib.IN_SUMS_ZEROED if zeroed else 0)
-    check(lib.ast_instnorm_bwd(ref(xi), ptr(mean), ptr(rstd), ptr(gamma), ptr(beta), ref(gp), pad, ref(ge), flags, ptr(s1),
-                               ptr(s2), ptr(arrive) if zeroed else None, ref(dxi), ref(gt), stream_ptr()), "ast_instnorm_bwd")
+    check(lib.ast_instnorm_bwd(ref(xi), ptr(mean), ptr(rstd), ptr(gamma), ptr(beta), ref(gp), pad, ref(ge), int(relu),
+                               ptr(s1), ptr(s2), ptr(arrive), ref(dxi), ref(gt), stream_ptr()), "ast_instnorm_bwd")
     return s12
 
 
@@ -373,13 +374,11 @@ def instnorm_apply(x, mean, rstd, gamma, beta, out, pad, relu, residual=None):
         return _instnorm_apply_impl(x, mean, rstd, gamma, beta, out, pad, relu, residual=residual)
 
 
-def instnorm_bwd(x, mean, rstd, gamma, beta, gpad, pad, gextra, relu, dx, gtotal=None, s12=None, zeroed=False, arrive=None):
-    """zeroed=True: `s12` (and `arrive`, n int32 barrier counters) were zero-filled by the caller: one fill for all layers
-    instead of two memsets per call, and the single-kernel backward (statistics + apply with the second read served from
-    L2) becomes available."""
+def instnorm_bwd(x, mean, rstd, gamma, beta, gpad, pad, gextra, relu, dx, gtotal=None, s12=None, arrive=None):
+    """`s12` and `arrive` (n int32 barrier counters), when given, are zero-filled by the caller: one fill for all layers."""
     with _timed("instnorm" + (f"|bwd{tuple(x.shape)}" if PROFILE_DETAIL and _prof is not None else "")):
         return _instnorm_bwd_impl(x, mean, rstd, gamma, beta, gpad, pad, gextra, relu, dx, gtotal=gtotal, s12=s12,
-                                  zeroed=zeroed, arrive=arrive)
+                                  arrive=arrive)
 
 
 def maxpool2_fwd(x, codes=None, out_dtype=None):

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define AST_ABI_VERSION 6
+#define AST_ABI_VERSION 7
 
 typedef enum {
   AST_F32 = 0, AST_BF16 = 1,
@@ -179,24 +179,13 @@ int ast_instnorm_apply(const ast_image* x, const float* mean, const float* rstd,
                        int32_t relu, void* stream);
 /* Backward of (ReflectionPad o ReLU o (+residual) o InstanceNorm).
  *   g'   = (fold_reflect(gpad, pad) + gextra) * (relu ? y>0 : 1)
- *   s1[n,c] = sum g' ; s2[n,c] = sum g'*xhat                       (pass 1, ast_instnorm_bwd_stats)
- *   dx   = gamma*rstd*(g' - s1/HW - xhat*s2/HW) ; gtotal = g'      (pass 2, ast_instnorm_bwd_apply)
- * gpad may be NULL (no padded consumer), gextra may be NULL, gtotal may be NULL.
- * relu: bit 0 = the forward applied ReLU; AST_IN_SUMS_ZEROED = s1/s2 were zeroed by the caller (one fill for all layers)
- * instead of two memsets per call. */
-#define AST_IN_SUMS_ZEROED 2
-int ast_instnorm_bwd_stats(const ast_image* x, const float* mean, const float* rstd, const float* gamma,
-                           const float* beta, const ast_image* gpad, int32_t pad, const ast_image* gextra,
-                           int32_t relu, float* s1, float* s2, void* stream);
-int ast_instnorm_bwd_apply(const ast_image* x, const float* mean, const float* rstd, const float* gamma,
-                           const float* beta, const ast_image* gpad, int32_t pad, const ast_image* gextra,
-                           int32_t relu, const float* s1, const float* s2, const ast_image* dx,
-                           const ast_image* gtotal, void* stream);
-
-/* Both passes in one call.  With `arrive` (n int32, ZERO on entry, together with AST_IN_SUMS_ZEROED) and x + g' small
- * enough to stay in the 126 MB L2, ONE cooperative kernel runs the statistics pass, meets the other blocks of the same
- * image at a counter barrier and re-reads its rows for the apply pass from L2 (5 HBM passes instead of 7); otherwise the
- * two kernels above run back to back.  Same results either way. */
+ *   s1[n,c] = sum g' ; s2[n,c] = sum g'*xhat                       (pass 1)
+ *   dx   = gamma*rstd*(g' - s1/HW - xhat*s2/HW) ; gtotal = g'      (pass 2)
+ * gpad may be NULL (no padded consumer), gextra may be NULL, gtotal may be NULL.  relu: 0 or 1 (the forward applied ReLU).
+ * s1, s2 (n*c floats) and arrive (n int32) must be ZERO on entry (one fill can serve every layer of a step).
+ * When x + g' are small enough to stay in the 126 MB L2, ONE cooperative kernel runs the statistics pass, meets the other
+ * blocks of the same image at a counter barrier (`arrive`) and re-reads its rows for the apply pass from L2 (5 HBM passes
+ * instead of 7); otherwise the two passes run as two launches.  Same results either way. */
 int ast_instnorm_bwd(const ast_image* x, const float* mean, const float* rstd, const float* gamma, const float* beta,
                      const ast_image* gpad, int32_t pad, const ast_image* gextra, int32_t relu, float* s1, float* s2,
                      int32_t* arrive, const ast_image* dx, const ast_image* gtotal, void* stream);

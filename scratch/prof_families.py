@@ -84,12 +84,12 @@ todo.append(("in_apply_staged bf16 64^2x128 +ReLU +reflect pad 1", lambda: ops.i
 s12 = torch.zeros(2, n * 128, device=dev); arr = torch.zeros(n, dtype=torch.int32, device=dev)
 def inb():
     s12.zero_(); arr.zero_()
-    ops.instnorm_bwd(xn, mean, rstd, gam, bet, gp, 1, None, True, dxn, None, s12=s12, zeroed=True, arrive=arr)
-todo.append(("in_bwd_fused_staged bf16 64^2x128 (stats + apply, one cooperative kernel)", inb))
+    ops.instnorm_bwd(xn, mean, rstd, gam, bet, gp, 1, None, True, dxn, None, s12=s12, arrive=arr)
+todo.append(("in_bwd_staged bf16 64^2x128 (stats + apply, one cooperative kernel)", inb))
 xb = torch.randn(n, 256, 256, 32, device=dev).to(bf); gpb = torch.randn(n, 264, 264, 32, device=dev).to(bf)
 mb = torch.randn(n * 32, device=dev); rb = torch.rand(n * 32, device=dev) + 0.5
 dxb = torch.empty_like(xb)
-todo.append(("in_bwd_stats_staged + in_bwd_apply_staged bf16 256^2x32 pad 4", lambda: ops.instnorm_bwd(xb, mb, rb, gam[:32].contiguous(), bet[:32].contiguous(), gpb, 4, None, True, dxb, None)))
+todo.append(("in_bwd_staged bf16 256^2x32 pad 4 (stats, then apply: two launches)", lambda: ops.instnorm_bwd(xb, mb, rb, gam[:32].contiguous(), bet[:32].contiguous(), gpb, 4, None, True, dxb, None)))
 # pointwise
 xp = torch.relu(torch.randn(n, 256, 256, 64, device=dev)); gy = torch.randn(n, 128, 128, 64, device=dev).to(bf)
 ga = torch.randn(n, 256, 256, 64, device=dev).to(bf)

@@ -19,18 +19,14 @@ def bench(n, h, w, c, pad, relu, residual, sets=6, iters=30):
     gam = torch.randn(c, device='cuda'); bet = torch.randn(c, device='cuda')
     s12 = torch.zeros(64, 2, n * c, device='cuda')
     arrive = torch.zeros(64, n, dtype=torch.int32, device='cuda')
-    def run_bwd(i):
+    def run_bwd(i):                 # zeroed sums / counters: a fresh slice per call
         x, gp, ge, dx, gt, out = bufs[i % sets]
-        ops._instnorm_bwd_impl(x, mean, rstd, gam, bet, gp, pad, ge, relu, dx, gtotal=gt)
-    def run_bwd_fused(i):           # single cooperative kernel (zeroed sums / counters: a fresh slice per call)
-        x, gp, ge, dx, gt, out = bufs[i % sets]
-        ops._instnorm_bwd_impl(x, mean, rstd, gam, bet, gp, pad, ge, relu, dx, gtotal=gt, s12=s12[i % 64], zeroed=True,
+        ops._instnorm_bwd_impl(x, mean, rstd, gam, bet, gp, pad, ge, relu, dx, gtotal=gt, s12=s12[i % 64],
                                arrive=arrive[i % 64])
     def run_apply(i):
         x, gp, ge, dx, gt, out = bufs[i % sets]
         ops._instnorm_apply_impl(x, mean, rstd, gam, bet, out, pad, relu, residual=ge)
     for name, fn, nbytes in (("bwd", run_bwd, (x.numel() * (2 + 1 + (2 if residual else 0)) + gp.numel() * 2) * 2),
-                             ("bwd1k", run_bwd_fused, (x.numel() * (2 + 1 + (2 if residual else 0)) + gp.numel() * 2) * 2),
                              ("apply", run_apply, (x.numel() * (1 + (1 if residual else 0)) + out.numel()) * 2)):
         for i in range(5): fn(i)
         torch.cuda.synchronize()

@@ -21,7 +21,7 @@ def test_header_symbols_exported():
     for n in names:
         assert hasattr(lib, n), f"{n} declared in include/ast.h but not exported by libast_b200.so"
     assert sorted(_lib.EXPORTS) == names, "ctypes binding and header disagree"
-    assert lib.ast_abi_version() == 6
+    assert lib.ast_abi_version() == 7
     assert lib.ast_instnorm_workspace_bytes(4, 128) > 0
     assert lib.ast_launch_count() >= 0
 
@@ -31,6 +31,27 @@ def test_argument_errors_are_loud():
     lib = _lib.load()
     rc = lib.ast_pack_weights(None, None, 1, 1, 1, 1, 1, None, 0, None)
     assert rc < 0 and b"null" in lib.ast_last_error()
+
+
+def test_instnorm_layouts_without_a_kernel_are_errors():
+    """InstanceNorm apply / backward run only on the staged kernels: mixed dtypes and a pixel stride other than C are
+    argument errors, reported before any CUDA call (the dummy pointers are never dereferenced)."""
+    from artist_style_transfer_b200 import _lib
+    lib = _lib.load()
+    n, h, w, c, pad = 2, 8, 8, 64, 1
+    p = ctypes.c_void_p(1 << 20)
+
+    def img(dtype, hh=h, ww=w, sw=c):
+        return _lib.Image(1 << 20, dtype, n, hh, ww, c, hh * ww * sw, ww * sw, sw, 1)
+    f32, bf16 = _lib.AST_F32, _lib.AST_BF16
+    for x, out, what in ((img(f32), img(bf16, h + 2, w + 2), b"dtype"),
+                         (img(bf16, sw=2 * c), img(bf16, h + 2, w + 2, sw=2 * c), b"dense")):
+        rc = lib.ast_instnorm_apply(ctypes.byref(x), p, p, p, p, None, ctypes.byref(out), pad, 1, None)
+        assert rc < 0 and what in lib.ast_last_error(), lib.ast_last_error()
+        dx = img(out.dtype, sw=2 * c if what == b"dense" else c)
+        rc = lib.ast_instnorm_bwd(ctypes.byref(x), p, p, p, p, ctypes.byref(out), pad, None, 1, p, p, p, ctypes.byref(dx),
+                                  None, None)
+        assert rc < 0 and what in lib.ast_last_error(), lib.ast_last_error()
 
 
 def test_no_cpu_fallback():

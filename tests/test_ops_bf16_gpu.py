@@ -35,53 +35,101 @@ def bf(x):
     return x.to(torch.bfloat16)
 
 
-@pytest.mark.parametrize("n,h,w,c,pad,relu,res", [(2, 64, 64, 128, 1, True, False), (2, 64, 64, 128, 1, False, True),
-                                                   (1, 128, 128, 64, 1, True, False), (1, 96, 80, 32, 4, True, False),
-                                                   (2, 64, 64, 128, 0, True, False)])
-@pytest.mark.parametrize("fused", [False, True])
-def test_instnorm_bwd_staged_bf16(env, n, h, w, c, pad, relu, res, fused):
-    """Backward of ReflectionPad o ReLU o (+residual) o InstanceNorm (cnn.py:58,68,91,98) on bf16 tensors: the two-kernel
-    path (statistics, apply) and the single cooperative kernel (second read from L2) give the same numbers."""
-    _lib, cg, ops = env
-    torch.manual_seed(c + h + pad)
-    x = bf(torch.randn(n, h, w, c, device="cuda") * 2 + 0.5)
-    gamma = torch.rand(c, device="cuda") + 0.5
-    beta = torch.randn(c, device="cuda") * 0.3
-    gpad = bf(torch.randn(n, h + 2 * pad, w + 2 * pad, c, device="cuda"))
-    gextra = bf(torch.randn(n, h, w, c, device="cuda")) if res else None
-    xd = x.double().cpu().permute(0, 3, 1, 2).requires_grad_(True)
-    gd, bd = gamma.double().cpu().requires_grad_(True), beta.double().cpu().requires_grad_(True)
+def instnorm_bwd_reference(x, gamma, beta, gpad, pad, gextra, relu):
+    """fp64 backward of ReflectionPad o ReLU o (+residual) o InstanceNorm on the device (CPU autograd at 10^8 elements is
+    too slow) -> fp32 mean / rstd, dbeta, dgamma, dx and g' (NHWC; g' only with gextra)."""
+    xd = x.double().permute(0, 3, 1, 2).requires_grad_(True)
+    gd, bd = gamma.double().requires_grad_(True), beta.double().requires_grad_(True)
     y = F.instance_norm(xd, weight=gd, bias=bd, eps=1e-5)
     if relu:
         y = F.relu(y)
     yp = F.pad(y, (pad,) * 4, mode="reflect") if pad else y
-    loss = (yp * gpad.double().cpu().permute(0, 3, 1, 2)).sum()
-    if res:
-        loss = loss + (y * gextra.double().cpu().permute(0, 3, 1, 2)).sum()
+    loss = (yp * gpad.double().permute(0, 3, 1, 2)).sum()
+    if gextra is not None:
+        loss = loss + (y * gextra.double().permute(0, 3, 1, 2)).sum()
     loss.backward()
-    mean = xd.detach().mean(dim=(2, 3)).reshape(-1).float().cuda()
-    rstd = (xd.detach().var(dim=(2, 3), unbiased=False) + 1e-5).rsqrt().reshape(-1).float().cuda()
+    mean = xd.detach().mean(dim=(2, 3)).reshape(-1).float()
+    rstd = (xd.detach().var(dim=(2, 3), unbiased=False) + 1e-5).rsqrt().reshape(-1).float()
+    gprime = None
+    if gextra is not None:
+        yr = F.instance_norm(xd.detach(), weight=gd.detach(), bias=bd.detach(), eps=1e-5)
+        gp = gpad.double().permute(0, 3, 1, 2)
+        fold = torch.autograd.functional.vjp(lambda t: F.pad(t, (pad,) * 4, mode="reflect") if pad else t, yr, gp)[1]
+        gprime = ((fold + gextra.double().permute(0, 3, 1, 2)) * ((yr > 0) if relu else 1.0)).permute(0, 2, 3, 1)
+    return mean, rstd, bd.grad, gd.grad, xd.grad.permute(0, 2, 3, 1), gprime
+
+
+@pytest.mark.parametrize("dt,n,h,w,c,pad,relu,res,launches", [
+    # x + g' small enough to stay in L2: one cooperative kernel
+    ("bf16", 2, 64, 64, 128, 1, True, False, 1), ("bf16", 2, 64, 64, 128, 1, False, True, 1),
+    ("bf16", 1, 128, 128, 64, 1, True, False, 1), ("bf16", 1, 96, 80, 32, 4, True, False, 1),
+    ("bf16", 2, 64, 64, 128, 0, True, False, 1), ("fp32", 2, 64, 64, 128, 1, True, False, 1),
+    # production layers too large for L2: statistics, then apply
+    ("bf16", 32, 128, 128, 64, 1, True, False, 2), ("bf16", 32, 256, 256, 32, 4, True, False, 2),
+    ("bf16", 16, 128, 128, 128, 1, False, True, 2), ("fp32", 32, 128, 128, 64, 1, True, False, 2)])
+def test_instnorm_bwd_staged_bf16(env, dt, n, h, w, c, pad, relu, res, launches):
+    """Backward of ReflectionPad o ReLU o (+residual) o InstanceNorm (cnn.py:58,68,91,98) against fp64 on the same rounded
+    operands, on both sides of the library's size rule: the single cooperative kernel (second read from L2) and the
+    two launches give the same numbers."""
+    _lib, cg, ops = env
+    torch.manual_seed(c + h + pad)
+    dtype = torch.bfloat16 if dt == "bf16" else torch.float32
+    x = (torch.randn(n, h, w, c, device="cuda") * 2 + 0.5).to(dtype)
+    gamma = torch.rand(c, device="cuda") + 0.5
+    beta = torch.randn(c, device="cuda") * 0.3
+    gpad = torch.randn(n, h + 2 * pad, w + 2 * pad, c, device="cuda").to(dtype)
+    gextra = torch.randn(n, h, w, c, device="cuda").to(dtype) if res else None
+    mean, rstd, dbeta, dgamma, dx_ref, gprime = instnorm_bwd_reference(x, gamma, beta, gpad, pad, gextra, relu)
     dx = torch.empty_like(x)
     gtotal = torch.empty_like(x) if res else None
+    s12 = torch.zeros(2, n * c, device="cuda")
+    arrive = torch.zeros(n, dtype=torch.int32, device="cuda")
     before = _lib.family_stats()
-    if fused:
-        s12 = torch.zeros(2, n * c, device="cuda")
-        arrive = torch.zeros(n, dtype=torch.int32, device="cuda")
-        ops.instnorm_bwd(x, mean, rstd, gamma, beta, gpad, pad, gextra, relu, dx, gtotal, s12=s12, zeroed=True, arrive=arrive)
-        assert _lib.family_delta(before)["in_bwd"][0] == 1, "single-kernel InstanceNorm backward expected"
+    ops.instnorm_bwd(x, mean, rstd, gamma, beta, gpad, pad, gextra, relu, dx, gtotal, s12=s12, arrive=arrive)
+    assert _lib.family_delta(before)["in_bwd"][0] == launches, f"{launches} InstanceNorm backward launch(es) expected"
+    if launches == 1:
         assert int(arrive.min()) == int(arrive.max()) > 0
-    else:
-        s12 = ops.instnorm_bwd(x, mean, rstd, gamma, beta, gpad, pad, gextra, relu, dx, gtotal)
-        assert _lib.family_delta(before)["in_bwd"][0] == 2, "staged InstanceNorm backward kernels expected"
-    assert rel(s12[0].view(n, c).sum(0), bd.grad) < 1e-5            # dbeta = sum g'
-    assert rel(s12[1].view(n, c).sum(0), gd.grad) < 2e-5            # dgamma = sum g' xhat
-    assert_bf16_close(dx, xd.grad.permute(0, 2, 3, 1), "dx")
+    assert rel(s12[0].view(n, c).sum(0), dbeta) < 1e-5              # dbeta = sum g'
+    assert rel(s12[1].view(n, c).sum(0), dgamma) < 2e-5             # dgamma = sum g' xhat
+    assert_bf16_close(dx, dx_ref, "dx")
     if res:        # gtotal = g' (the gradient handed to the residual skip)
-        yr = F.instance_norm(xd.detach(), weight=gd.detach(), bias=bd.detach(), eps=1e-5)
-        gp = gpad.double().cpu().permute(0, 3, 1, 2)
-        fold = torch.autograd.functional.vjp(lambda t: F.pad(t, (pad,) * 4, mode="reflect") if pad else t, yr, gp)[1]
-        gprime = (fold + gextra.double().cpu().permute(0, 3, 1, 2)) * ((yr > 0) if relu else 1.0)
-        assert_bf16_close(gtotal, gprime.permute(0, 2, 3, 1), "gtotal")
+        assert_bf16_close(gtotal, gprime, "gtotal")
+
+
+def test_instnorm_images_more_than_2g_elements_apart(env):
+    """Strict-mode batches can span more than 2^31 elements: the staged InstanceNorm kernels address image and row starts
+    in 64 bits.  Two images 2^31 + 1024 elements apart (views into one 4.3 GB buffer): the apply output is bit-identical
+    to the one computed from compact copies, and the backward meets the fp64 bounds of the test above."""
+    _lib, cg, ops = env
+    torch.manual_seed(7)
+    n, h, w, c, pad = 2, 64, 64, 128, 1
+    hp, wp = h + 2 * pad, w + 2 * pad
+    sn = 2 ** 31 + 1024
+    big = torch.empty(sn + 4 * h * w * c + 2 * hp * wp * c, dtype=torch.bfloat16, device="cuda")
+    off = 0
+
+    def view(hh, ww):        # per image: x | residual | dx | gtotal | gpad | out, the images sn elements apart
+        nonlocal off
+        v = big.as_strided((n, hh, ww, c), (sn, ww * c, c, 1), off)
+        off += hh * ww * c
+        return v
+    x, res, dx, gtotal, gpad, out = view(h, w), view(h, w), view(h, w), view(h, w), view(hp, wp), view(hp, wp)
+    for t in (x, res, gpad):
+        t.copy_(torch.randn(t.shape, device="cuda"))
+    gamma = torch.rand(c, device="cuda") + 0.5
+    beta = torch.randn(c, device="cuda") * 0.3
+    mean, rstd, dbeta, dgamma, dx_ref, gprime = instnorm_bwd_reference(x, gamma, beta, gpad, pad, res, True)
+
+    ops.instnorm_apply(x, mean, rstd, gamma, beta, out, pad, True, residual=res)
+    out_c = torch.empty(out.shape, dtype=out.dtype, device="cuda")
+    ops.instnorm_apply(x.contiguous(), mean, rstd, gamma, beta, out_c, pad, True, residual=res.contiguous())
+    assert torch.equal(out, out_c)
+
+    s12 = ops.instnorm_bwd(x, mean, rstd, gamma, beta, gpad, pad, res, True, dx, gtotal)
+    assert rel(s12[0].view(n, c).sum(0), dbeta) < 1e-5
+    assert rel(s12[1].view(n, c).sum(0), dgamma) < 2e-5
+    assert_bf16_close(dx, dx_ref, "dx")
+    assert_bf16_close(gtotal, gprime, "gtotal")
 
 
 def test_maxpool2_bwd_and_mask_add_bf16(env):
