@@ -98,6 +98,7 @@ _SIGNATURES = {
     "ast_channel_sum": [_P(Image), _vp, _vp],
     "ast_mse": [_P(Image), _P(Image), _vp, ctypes.c_float, _P(Image), ctypes.c_float, _vp],
     "ast_copy_image": [_P(Image), _P(Image), _vp, ctypes.c_int32, _vp],
+    "ast_reflect_fold": [_P(Image), _P(Image), _P(Image), ctypes.c_int32, _vp],
     "ast_accumulate": [_P(Image), _P(Image), _vp],
     "ast_mask_add": [_P(Image), _P(Image), _P(Image), _P(Image), _vp],
 }

@@ -95,11 +95,67 @@ class _StagePlan:
     __slots__ = ("thin_in", "thin_out", "fwd", "dgrad", "g_shape", "g_taps", "g_stride", "g_off", "g_cb", "g_gam", "g_bet")
 
 
+def thin_in_dgrad_taps(k):
+    """(taps, wtaps) of the data gradient of a thin-input stage, w.r.t. its reflect-padded cin-channel image P:
+    part[n, Y, x, d*cin + c] = sum_{u, co} dY[n, Y - u, x - (k-1), co] * W[co, c, u, k-1-d] over a (h+2p, w+2(k-1)) grid,
+    and ast_fold_rows then gives gP[n, Y, X, c] = sum_d part[n, Y, X + d, d*cin + c]."""
+    return [(-u, -(k - 1)) for u in range(k)], [(u, 0) for u in range(k)]
+
+
+def dgrad_pack(st, pl, tc, adt):
+    """Layout of the data-gradient operand copy of one stage's filter.  The arena holds it for every stage but the first;
+    TransferArena.stage0_dgrad builds the first stage's from the same layout when an input gradient is asked for."""
+    k, co, ci = st.k, st.cout, st.cin
+    conv = st.kind == "conv"
+    uv = [(u, v) for u in range(k) for v in range(k)]
+    if pl.thin_in:        # [u][d*cin + c][co] (k, 32, cout): a thin-output conv of dY, see thin_in_dgrad_taps
+        taps, wt = thin_in_dgrad_taps(k)
+        if (co * 2) % 128 == 0 or co * 2 == 64:
+            vt = [cg.Launch(16, 16, 1, 1, 0, 0, taps, wt, 0)]
+            return _stacked_pack(stack_groups(vt, 32), 32, co, adt, uv, lambda u, v: (u, 0),
+                                 lambda u, v: (k - 1 - v) * ci * co, (1, co))
+        return _Pack((k, 32, co), adt, [u * 32 * co + (k - 1 - v) * ci * co for u, v in uv], (1, co))
+    if pl.thin_out:       # [dy][c][dx*cout + co] (k, cin, 32)
+        if ci == 32:      # block-stacked: rows y - dy of the row-im2col'd output gradient
+            vt_dg = [cg.Launch(16, 16, 1, 1, 0, 0, [(-u, 0) for u in range(k)], [(u, 0) for u in range(k)], 0)]
+            return _stacked_pack(stack_groups(vt_dg, ci), ci, 32, adt, uv, lambda u, v: (u, 0), lambda u, v: v * co,
+                                 (1, 32))
+        return _Pack((k, ci, 32), adt, [u * ci * 32 + v * co for u, v in uv], (1, 32))
+    # [t][ci][co], t in the order of the data-gradient launches' taps (phases for stride 2)
+    canon = _canonical_dgrad(st)
+    dg_stride = (1, co) if conv else (co, 1)
+    if tc and conv and st.stride == 2 and ci in (32, 64) and (co * 2) % 128 == 0:
+        # data gradient of a stride-2 conv: the 4 output phases as lane blocks
+        return _stacked_pack(stack_groups(canon, ci), ci, co, adt, uv, lambda u, v: (u, v), lambda u, v: 0, dg_stride)
+    order = cg.all_wtaps(canon)
+    tapidx = {t: n for n, t in enumerate(order)}
+    return _Pack((k * k, ci, co), adt, [tapidx[t] * ci * co for t in uv], dg_stride, tapidx)
+
+
+def _param_desc(p_off, s_off, dims, g_off, g_stride, g_tap, packs, add_taps):
+    """ast_param_desc of one parameter tensor; add_taps(list) -> first index of `list` in the tap table."""
+    d = ParamDesc()
+    d.p_off, d.s_off = p_off, s_off
+    numel = 1
+    for n_, v in enumerate(dims):
+        d.dim[n_] = v
+        numel *= v
+    d.numel = numel
+    d.g_off, d.g_tap, d.n_pack = g_off, g_tap, len(packs)
+    d.g_stride[0], d.g_stride[1] = g_stride
+    for n_, pk in enumerate(packs):
+        d.pack[n_].off, d.pack[n_].tap, d.pack[n_].dtype = pk.off, add_taps(pk.taps), _DT_CODE[pk.dtype]
+        d.pack[n_].stride[0], d.pack[n_].stride[1] = pk.stride
+        d.pack[n_].rep, d.pack[n_].rep_stride = pk.rep, pk.rep_stride
+    return d
+
+
 class TransferArena:
     def __init__(self, stages, mode, device, thin_in_ok=True):
         self.stages, self.mode, self.device = list(stages), mode, device
         self.adt = torch.bfloat16 if mode == "fast" else torch.float32
         tc = mode == "fast" and _lib.has_tc_conv()
+        self.tc = tc
         self.plans = []
         goff = 0
 
@@ -146,26 +202,8 @@ class TransferArena:
                     pl.fwd = _Pack((k2, co, ci), self.adt, [tapidx[t] * co * ci for t in uv], sa_sb, tapidx)
                 # tap-major gradient scratch [u][v][co][ci]: ci contiguous -> 16-byte vector reductions in the epilogue
                 pl.g_shape, pl.g_taps, pl.g_stride = (k, k, co, ci), [(u * k + v) * co * ci for u, v in uv], sa_sb
-            pl.dgrad = None
-            if i > 0:
-                if pl.thin_out:   # [dy][c][dx*cout + co] (k, cin, 32)
-                    if ci == 32:  # block-stacked: rows y - dy of the row-im2col'd output gradient
-                        vt_dg = [cg.Launch(16, 16, 1, 1, 0, 0, [(-u, 0) for u in range(k)], [(u, 0) for u in range(k)], 0)]
-                        pl.dgrad = _stacked_pack(stack_groups(vt_dg, ci), ci, 32, self.adt, uv, lambda u, v: (u, 0),
-                                                 lambda u, v: v * co, (1, 32))
-                    else:
-                        pl.dgrad = _Pack((k, ci, 32), self.adt, [u * ci * 32 + v * co for u, v in uv], (1, 32))
-                else:             # [t][ci][co], t in the order of the data-gradient launches' taps (phases for stride 2)
-                    canon = _canonical_dgrad(st)
-                    dg_stride = (1, co) if conv else (co, 1)
-                    if tc and conv and st.stride == 2 and ci in (32, 64) and (co * 2) % 128 == 0:
-                        # data gradient of a stride-2 conv: the 4 output phases as lane blocks
-                        pl.dgrad = _stacked_pack(stack_groups(canon, ci), ci, co, self.adt, uv, lambda u, v: (u, v),
-                                                 lambda u, v: 0, dg_stride)
-                    else:
-                        order = cg.all_wtaps(canon)
-                        tapidx = {t: n for n, t in enumerate(order)}
-                        pl.dgrad = _Pack((k2, ci, co), self.adt, [tapidx[t] * ci * co for t in uv], dg_stride, tapidx)
+            # the first stage's input gradient is optional: its pack is built on demand (stage0_dgrad)
+            pl.dgrad = dgrad_pack(st, pl, tc, self.adt) if i > 0 else None
             n = 1
             for d in pl.g_shape:
                 n *= d
@@ -191,6 +229,7 @@ class TransferArena:
         self._packs_key = None
         self.opt = None            # Adam state once enable_optimizer() was called
         self._reduce_cache = {}
+        self._dg0_tables = None    # (weight address, descriptor, work list, work items, tap table) of stage0_dgrad
 
     # ------------------------------------------------------------------ parameters
     def params(self):
@@ -221,19 +260,9 @@ class TransferArena:
 
         def add_desc(p, dims, g_off, g_stride, g_tap, packs):
             nonlocal s_off
-            d = ParamDesc()
             assert (p.data_ptr() - base) % 4 == 0
-            d.p_off, d.s_off, d.numel = (p.data_ptr() - base) // 4, s_off, p.numel()
-            for n_, v in enumerate(dims):
-                d.dim[n_] = v
-            d.g_off, d.g_tap, d.n_pack = g_off, g_tap, len(packs)
-            d.g_stride[0], d.g_stride[1] = g_stride
-            for n_, pk in enumerate(packs):
-                d.pack[n_].off, d.pack[n_].tap, d.pack[n_].dtype = pk.off, add_taps(pk.taps), _DT_CODE[pk.dtype]
-                d.pack[n_].stride[0], d.pack[n_].stride[1] = pk.stride
-                d.pack[n_].rep, d.pack[n_].rep_stride = pk.rep, pk.rep_stride
             idx = len(descs)
-            descs.append(d)
+            descs.append(_param_desc((p.data_ptr() - base) // 4, s_off, dims, g_off, g_stride, g_tap, packs, add_taps))
             for start in range(0, p.numel(), item):
                 work.append((idx, start))
             s_off += (p.numel() + 3) // 4 * 4
@@ -284,6 +313,39 @@ class TransferArena:
                                      _lib.ptr(o["v"]) if update else None, vp(self.pack_arena.data_ptr()),
                                      vp(self.taps_dev.data_ptr()), _lib.ptr(o["state"]) if update else None,
                                      1 if update else 0, _lib.stream_ptr()), "ast_adam_step")
+
+    def stage0_dgrad(self):
+        """The first stage's data-gradient filter (dgrad_pack layout, outside the pack arena), written from the current
+        weights by one ast_adam_step(update=0) launch over a one-descriptor table: the arena's packing code, stacked
+        replicas included.  Written on every call, never cached: the fused Adam updates the parameters in place without
+        bumping their versions, and a CUDA graph that captures the backward must capture this launch with it.  Only the
+        device tables are kept (they depend on the weight's address, not its values)."""
+        st, pl = self.stages[0], self.plans[0]
+        w = st.conv.weight
+        pk = dgrad_pack(st, pl, self.tc, self.adt)
+        t = self._dg0_tables
+        if t is None or t[0] != w.data_ptr():
+            if w.dtype != torch.float32 or not w.is_contiguous():
+                raise RuntimeError("TransformerNet master parameters must be contiguous fp32 tensors")
+            taps = []
+
+            def add_taps(lst):
+                taps.extend(int(x) for x in lst)
+                return 0
+            d = _param_desc(0, 0, tuple(w.shape), 0, (0, 0), 0, [pk], add_taps)
+            item = _lib.load().ast_adam_work_item()
+            work = [x for s in range(0, w.numel(), item) for x in (0, s)]
+            t = (w.data_ptr(), _lib.device_bytes(d, self.device),
+                 _lib.device_bytes((ctypes.c_int32 * len(work))(*work), self.device), len(work) // 2,
+                 torch.tensor(taps, dtype=torch.int64, device=self.device))
+            self._dg0_tables = t
+        buf = torch.zeros(pk.nbytes(), dtype=torch.uint8, device=self.device)   # zero rows of the stacked layouts
+        vp = ctypes.c_void_p
+        _lib.check(_lib.load().ast_adam_step(vp(t[1].data_ptr()), 1, vp(t[2].data_ptr()), t[3], _lib.ptr(w), None, None,
+                                             None, vp(buf.data_ptr()), vp(t[4].data_ptr()), None, 0, _lib.stream_ptr()),
+                   "ast_adam_step")
+        pk.tensor = buf.view(pk.dtype).view(pk.shape)
+        return pk
 
     def woff(self, pack, launches):
         """Rewrite each launch's first-tap index for the canonical tap order of `pack` (robust to skipped phases)."""

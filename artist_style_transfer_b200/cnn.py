@@ -115,6 +115,7 @@ class _StageFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, arena, nhwc, u8_out, *params):
         stages, mode, adt = arena.stages, arena.mode, arena.adt
+        x_shape, x_dtype = x.shape, x.dtype
         x = x.detach()
         if x.dtype not in (torch.float32, torch.uint8):
             x = x.to(torch.float32)
@@ -216,6 +217,7 @@ class _StageFunction(torch.autograd.Function):
                 xin = None
         if train:
             ctx.arena, ctx.P = arena, P
+            ctx.x_shape, ctx.x_dtype, ctx.nhwc = x_shape, x_dtype, nhwc
             ctx.nodes, ctx.node_pad, ctx.saved = nodes, node_pad, saved
         return out
 
@@ -223,9 +225,7 @@ class _StageFunction(torch.autograd.Function):
     def backward(ctx, gout):
         arena, P, nodes, node_pad, saved = ctx.arena, ctx.P, ctx.nodes, ctx.node_pad, ctx.saved
         stages, plans, mode = arena.stages, arena.plans, arena.mode
-        if ctx.needs_input_grad[0]:
-            raise NotImplementedError("gradient w.r.t. the input image is not part of the training path "
-                                      "(train_cnn.py:298-299 feeds data that does not require grad)")
+        want_gx = ctx.needs_input_grad[0]
         adt = nodes[0].dtype
         gdt = adt                                   # dtype of the gradients flowing between layers
         gout = gout.to(torch.float32)
@@ -298,31 +298,53 @@ class _StageFunction(torch.autograd.Function):
                 # vector atomics; the optimizer / p.grad read it through strides
                 ops.wgrad_gather(xin, d_raw, launches, g_w, st.cin, 1, st.k * st.cout * st.cin, st.cout * st.cin,
                                  tensor=wtc)
-            if i > 0 and pl.thin_out:
+            if i == 0 and not want_gx:
+                continue
+            # data gradient w.r.t. node i (stage 0: its pack is built now, outside the arena)
+            pk = pl.dgrad if i > 0 else arena.stage0_dgrad()
+            if i == 0 and pl.thin_in:
+                # gradient w.r.t. the reflect-padded 3-channel image as a 32 -> 3 k x k conv of d_raw in the last layer's
+                # thin-output form: k vertical taps into k*cin partial channels, then ast_fold_rows
+                k, p = st.k, st.in_pad
+                n, h, w = d_raw.shape[:3]
+                taps, wt = arena_mod.thin_in_dgrad_taps(k)
+                part = torch.empty((n, h + 2 * p, w + 2 * (k - 1), 32), dtype=torch.float32, device=dev)
+                _conv_packed(d_raw, pk, [cg.Launch(h + 2 * p, w + 2 * (k - 1), 1, 1, 0, 0, taps, wt, 0)], part, tensor=True)
+                g_in = torch.empty((n, h + 2 * p, w + 2 * p, st.cin), dtype=torch.float32, device=dev)
+                ops.fold_rows(part, g_in, k)
+                del part
+            elif pl.thin_out:
                 taps, wt = _vtaps(st.k, -1)
                 dl = [cg.Launch(xin.shape[1], xin.shape[2], 1, 1, 0, 0, taps, wt, 0)]
                 g_in = torch.empty(xin.shape, dtype=gdt, device=dev)
-                _conv_packed(d_raw, pl.dgrad, dl, g_in, tensor=True)
-                gpad[i] = g_in
-            elif i > 0:
+                _conv_packed(d_raw, pk, dl, g_in, tensor=True)
+            else:
                 if st.kind == "conv":
                     dl = cg.conv_dgrad(st.k, st.stride, 0, xin.shape[1], xin.shape[2])
                 else:
                     dl = cg.convT_dgrad(st.k, st.stride, st.k // 2, d_raw.shape[1], d_raw.shape[2])
-                arena.woff(pl.dgrad, dl)
+                arena.woff(pk, dl)
                 g_in = torch.empty(xin.shape, dtype=gdt, device=dev)
                 src = d_raw
                 if src.dtype != adt or not src.is_contiguous():   # fp32 NCHW grad of the last conv feeding the dgrad
                     src = torch.empty(d_raw.shape, dtype=adt, device=dev)
                     ops.copy_image(d_raw, src)
-                _conv_packed(src, pl.dgrad, dl, g_in, tensor=mode == "fast" and ops.tc_eligible(src, st.cin))
-                gpad[i] = g_in
+                _conv_packed(src, pk, dl, g_in, tensor=mode == "fast" and ops.tc_eligible(src, st.cin))
+            gpad[i] = g_in
+        gx = None
+        if want_gx:
+            # adjoint of how the forward wrote the input into node 0, plus the skip gradient of a standalone
+            # ResidualLayer (node 0's interior is also its residual)
+            gx = torch.empty(ctx.x_shape, dtype=ctx.x_dtype if ctx.x_dtype == torch.bfloat16 else torch.float32,
+                             device=dev)
+            ops.reflect_fold(gpad[0], gx if ctx.nhwc else gx.permute(0, 2, 3, 1), node_pad[0], add=gextra[0])
+            gx = gx.to(ctx.x_dtype)
         if bank_off:
             ops.batch_reduce(banks, gbuf, *arena.reduce_table(nb, bank_off))
         ctx.nodes = ctx.saved = None
         if sink is not None:                         # the trainer reads the arena directly (p.grad are views of it)
-            return (None,) * (4 + len(arena.params()))
-        return (None, None, None, None, *arena.grad_views(gbuf))
+            return (gx,) + (None,) * (3 + len(arena.params()))
+        return (gx, None, None, None, *arena.grad_views(gbuf))
 
 
 class _Precision:

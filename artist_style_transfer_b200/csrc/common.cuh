@@ -134,6 +134,27 @@ __device__ __forceinline__ int reflect_idx(int i, int n) {
   if (i >= n) i = 2 * (n - 1) - i;
   return i;
 }
+// Adjoint of reflect padding by pad < H, W: besides the centre (i + pad, j + pad), the positions (r, c) of the
+// (H+2pad) x (W+2pad) grid that reflect_idx maps onto interior pixel (i, j).  add(r, c) is called for each of them in a
+// fixed order (rows: centre, top mirror, bottom mirror; columns likewise), so every caller sums in the same order.
+template <typename F>
+__device__ __forceinline__ void reflect_fold_border(int pad, int H, int W, int i, int j, F&& add) {
+  const int r1 = (i >= 1 && i <= pad) ? pad - i : -1;
+  const int r2 = (i <= H - 2 && i >= H - 1 - pad) ? pad + 2 * (H - 1) - i : -1;
+  const int c1 = (j >= 1 && j <= pad) ? pad - j : -1;
+  const int c2 = (j <= W - 2 && j >= W - 1 - pad) ? pad + 2 * (W - 1) - j : -1;
+#pragma unroll
+  for (int a_ = 0; a_ < 3; ++a_) {
+    const int r = a_ == 0 ? i + pad : (a_ == 1 ? r1 : r2);
+    if (r < 0) continue;
+#pragma unroll
+    for (int b_ = 0; b_ < 3; ++b_) {
+      const int cc = b_ == 0 ? j + pad : (b_ == 1 ? c1 : c2);
+      if (cc < 0 || (a_ == 0 && b_ == 0)) continue;
+      add(r, cc);
+    }
+  }
+}
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

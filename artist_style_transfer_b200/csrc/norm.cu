@@ -293,24 +293,12 @@ in_apply_staged_kernel(Rows x, const float* __restrict__ mean, const float* __re
 // gimg: channel c of pixel (0, 0) of this image of gpad, gsh: its row stride
 template <typename T, int VEC>
 __device__ __forceinline__ void ns_fold_border(const T* gimg, int gsh, int C, int pad, int H, int W, int i, int j, float* g) {
-  const int r1 = (i >= 1 && i <= pad) ? pad - i : -1;
-  const int r2 = (i <= H - 2 && i >= H - 1 - pad) ? pad + 2 * (H - 1) - i : -1;
-  const int c1 = (j >= 1 && j <= pad) ? pad - j : -1;
-  const int c2 = (j <= W - 2 && j >= W - 1 - pad) ? pad + 2 * (W - 1) - j : -1;
+  reflect_fold_border(pad, H, W, i, j, [&](int r, int cc) {
+    float t[VEC];
+    NsVec<T>::unpack(__ldg(reinterpret_cast<const uint4*>(gimg + (r * gsh + cc * C))), t);
 #pragma unroll
-  for (int a_ = 0; a_ < 3; ++a_) {
-    const int r = a_ == 0 ? i + pad : (a_ == 1 ? r1 : r2);
-    if (r < 0) continue;
-#pragma unroll
-    for (int b_ = 0; b_ < 3; ++b_) {
-      const int cc = b_ == 0 ? j + pad : (b_ == 1 ? c1 : c2);
-      if (cc < 0 || (a_ == 0 && b_ == 0)) continue;
-      float t[VEC];
-      NsVec<T>::unpack(__ldg(reinterpret_cast<const uint4*>(gimg + (r * gsh + cc * C))), t);
-#pragma unroll
-      for (int e = 0; e < VEC; ++e) g[e] += t[e];
-    }
-  }
+    for (int e = 0; e < VEC; ++e) g[e] += t[e];
+  });
 }
 
 // producer of the backward: x row segment, the centre of the padded gradient row, the extra gradient, for this block's

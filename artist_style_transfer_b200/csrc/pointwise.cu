@@ -1,7 +1,8 @@
 // HBM-bound elementwise / reduction kernels of the path: max-pool (fwd, bwd fused with tap-gradient add and
-// ReLU mask), MSE (loss + gradient seed), layout/dtype copies, feature accumulation, Gram (SIMT).
+// ReLU mask), MSE (loss + gradient seed), layout/dtype copies and the reflect-padding adjoint, feature accumulation,
+// Gram (SIMT).
 // Replaces aten::max_pool2d_with_indices(+backward), aten::threshold_backward, aten::mse_loss(+backward),
-// aten::add_ / aten::add at train_cnn.py:54,239,300-301,307,323.
+// aten::add_ / aten::add at train_cnn.py:54,239,300-301,307,323, aten::reflection_pad2d_backward at cnn.py:58.
 #include "common.cuh"
 
 namespace ast {
@@ -184,6 +185,22 @@ __global__ void __launch_bounds__(NT) copy_image_kernel(Img src, Img dst, const 
       if (shift) v += shift[c];
     }
     st_elem(dst, img_off(dst, n, y, x, c), v);
+  }
+}
+
+// adjoint of copy_image_kernel's reflect padding: one thread per output element, in the output's fastest-varying order
+__global__ void __launch_bounds__(NT) reflect_fold_kernel(Img gpad, Img add, Img out, int pad) {
+  const long long total = (long long)out.n * out.h * out.w * out.c;
+  const bool chan_fast = out.sc == 1;
+  for (long long idx = blockIdx.x * (long long)NT + threadIdx.x; idx < total; idx += (long long)gridDim.x * NT) {
+    int n, y, x, c;
+    long long r = idx;
+    if (chan_fast) { c = (int)(r % out.c); r /= out.c; x = (int)(r % out.w); r /= out.w; y = (int)(r % out.h); n = (int)(r / out.h); }
+    else { x = (int)(r % out.w); r /= out.w; y = (int)(r % out.h); r /= out.h; c = (int)(r % out.c); n = (int)(r / out.c); }
+    float v = ld_elem(gpad, img_off(gpad, n, y + pad, x + pad, c));
+    reflect_fold_border(pad, out.h, out.w, y, x, [&](int yy, int xx) { v += ld_elem(gpad, img_off(gpad, n, yy, xx, c)); });
+    if (add.ptr) v += ld_elem(add, img_off(add, n, y, x, c));
+    st_elem(out, img_off(out, n, y, x, c), v);
   }
 }
 
@@ -384,6 +401,26 @@ extern "C" int ast_copy_image(const ast_image* src, const ast_image* dst, const 
   launch_k(copy_image_kernel, blocks_for(total), NT, 0, (cudaStream_t)stream, to_img(src), to_img(dst), shift, pad);
   count_launch();
   count_work(FAM_POINTWISE, 0.0, img_bytes(src) + img_bytes(dst));
+  AST_CUDA_LAUNCH_CHECK();
+  return 0;
+}
+
+static bool f32_or_bf16(const ast_image* x) { return x->dtype == AST_F32 || x->dtype == AST_BF16; }
+
+extern "C" int ast_reflect_fold(const ast_image* gpad, const ast_image* add, const ast_image* out, int32_t pad, void* stream) {
+  AST_CHECK_ARG(gpad && out, "ast_reflect_fold: null argument");
+  AST_CHECK_ARG(f32_or_bf16(gpad) && f32_or_bf16(out) && (!add || f32_or_bf16(add)),
+                "ast_reflect_fold: gpad, add and out must be fp32 or bf16");
+  AST_CHECK_ARG(pad >= 0 && pad < out->h && pad < out->w, "ast_reflect_fold: pad must be >= 0 and < h, w");
+  AST_CHECK_ARG(gpad->n == out->n && gpad->c == out->c && gpad->h == out->h + 2 * pad && gpad->w == out->w + 2 * pad,
+                "ast_reflect_fold: gpad must be (n, h+2p, w+2p, c) of out");
+  AST_CHECK_ARG(!add || same_shape(add, out), "ast_reflect_fold: add must be shaped like out");
+  const long long total = (long long)out->n * out->h * out->w * out->c;
+  if (total == 0) return 0;
+  launch_k(reflect_fold_kernel, blocks_for(total), NT, 0, (cudaStream_t)stream, to_img(gpad), add ? to_img(add) : null_img(),
+           to_img(out), pad);
+  count_launch();
+  count_work(FAM_POINTWISE, 0.0, img_bytes(gpad) + img_bytes(add) + img_bytes(out));
   AST_CUDA_LAUNCH_CHECK();
   return 0;
 }

@@ -445,6 +445,14 @@ def copy_image(src, dst, shift=None, pad=0, flip_channels=False):
         return _copy_image_impl(src, dst, shift=shift, pad=pad, flip_channels=flip_channels)
 
 
+def reflect_fold(gpad, out, pad, add=None):
+    """out = adjoint of copy_image(..., pad) applied to gpad (+ add); see include/ast.h ast_reflect_fold."""
+    with _timed(_pw("reflect_fold", out)):
+        gi, ai, oi = image(gpad), image(add), image(out)
+        check(_lib.load().ast_reflect_fold(ref(gi), ref(ai), ref(oi), pad, stream_ptr()), "ast_reflect_fold")
+        return out
+
+
 def accumulate(x, acc):
     with _timed(_pw("accumulate", x)):
         return _accumulate_impl(x, acc)

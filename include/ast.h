@@ -222,6 +222,12 @@ int ast_mse(const ast_image* a, const ast_image* b, float* loss, float scale, co
 
 /* dst = src converted/re-strided (NCHW fp32 <-> NHWC bf16/fp32), optional per-channel shift, reflect pad. */
 int ast_copy_image(const ast_image* src, const ast_image* dst, const float* shift, int32_t pad, void* stream);
+/* Adjoint of ast_copy_image's reflect padding (aten::reflection_pad2d_backward of cnn.py:58): the gradient of a layer's
+ * input from the gradient of its reflection-padded copy,
+ *   out[n,i,j,c] = sum over (y,x) of the (h+2p) x (w+2p) grid with R(y-p) = i, R(x-p) = j of gpad[n,y,x,c]  (+ add[n,i,j,c])
+ * R = nn.ReflectionPad2d's index rule.  gpad: [n, h+2*pad, w+2*pad, c]; add: optional, shaped like out.  Each of gpad,
+ * add and out is fp32 or bf16 with any strides (e.g. an NCHW out view).  0 <= pad < h, w; pad = 0 is a conversion (+ add). */
+int ast_reflect_fold(const ast_image* gpad, const ast_image* add, const ast_image* out, int32_t pad, void* stream);
 /* acc(fp32 image) += x   ('smartaverage' in-place feature sum, train_cnn.py:239).  With acc->n == 1 and x->n > 1 the batch
  * of x is summed into the one accumulator image (several paintings per VGG pass). */
 int ast_accumulate(const ast_image* x, const ast_image* acc, void* stream);
