@@ -356,7 +356,7 @@ __device__ __forceinline__ void ns_gprime(unsigned xs, unsigned gs, unsigned es,
 enum NsMode { NS_STATS = 1, NS_APPLY = 2, NS_BOTH = 3 };
 
 // Backward of pad o ReLU o (+residual) o InstanceNorm, by MODE:
-//   NS_STATS  pass 1: s1[n,c] += sum g', s2[n,c] += sum g' * xhat
+//   NS_STATS  pass 1: s1[n,c] += sum g', s2[n,c] += rstd * sum g' * (x - mean) = sum g' * xhat
 //   NS_APPLY  pass 2: dx = A*g' + B*x + C (and gtotal = g') from the finished s1 / s2
 //   NS_BOTH   both passes in one cooperative launch.  Two launches read x and g' twice from HBM (7 physical passes for 5
 //             algorithmic ones).  For layers whose x + g' fit in the 126 MB L2 this kernel runs the statistics pass, meets
@@ -418,13 +418,16 @@ in_bwd_staged_kernel(Rows x, const float* __restrict__ mean, const float* __rest
   };
 
   if (MODE & NS_STATS) {
-    float t1[VEC], t2[VEC];
+    // sum g' * (x - mean), centred per element: a sum of g' * x corrected by mean * sum g' afterwards loses |mean| / std
+    // digits to cancellation, so its error would scale with sum |g'| * |x| instead of sum |g' * xhat|
+    float t1[VEC], t2[VEC], mu[VEC];
+    ns_ldc<VEC>(mean + n * C + c, mu);
 #pragma unroll
     for (int e = 0; e < VEC; ++e) { t1[e] = 0.f; t2[e] = 0.f; }
     for (int k = 0; k < nunits; ++k)
       consume(k, k, [&](int, const float* xv, const float* g) {
 #pragma unroll
-        for (int e = 0; e < VEC; ++e) { t1[e] += g[e]; t2[e] = fmaf(g[e], xv[e], t2[e]); }
+        for (int e = 0; e < VEC; ++e) { t1[e] += g[e]; t2[e] = fmaf(g[e], xv[e] - mu[e], t2[e]); }
       });
     // block reduction.  NS_STATS: in the ring, once every consumer warp has consumed every stage.  NS_BOTH: in a scratch
     // area BEHIND the ring (the producer is already refilling the ring for pass 2).
@@ -442,7 +445,7 @@ in_bwd_staged_kernel(Rows x, const float* __restrict__ mean, const float* __rest
       float u1 = 0.f, u2 = 0.f;
       for (int q = 0; q < slots; ++q) { u1 += r1[q * C + cc]; u2 += r2[q * C + cc]; }
       atomicAdd(s1 + n * C + cc, u1);
-      atomicAdd(s2 + n * C + cc, rstd[n * C + cc] * (u2 - mean[n * C + cc] * u1));
+      atomicAdd(s2 + n * C + cc, rstd[n * C + cc] * u2);
     }
     if (MODE == NS_BOTH) {
       // all blocks of image n have added their sums: release / acquire through the fence + counter

@@ -34,21 +34,26 @@ def test_argument_errors_are_loud():
 
 
 def test_instnorm_layouts_without_a_kernel_are_errors():
-    """InstanceNorm apply / backward run only on the staged kernels: mixed dtypes and a pixel stride other than C are
-    argument errors, reported before any CUDA call (the dummy pointers are never dereferenced)."""
+    """InstanceNorm apply / backward run only on the staged kernels: mixed dtypes, a pixel stride other than C, a C the
+    256 consumer threads cannot split into lanes (bf16 C=24: 3 lanes) and a pad whose mirrored border does not fit a row
+    segment (bf16 C=1024: 8 pixels per 16 KB segment, pad 4) are argument errors, reported before any CUDA call (the
+    dummy pointers are never dereferenced)."""
     from artist_style_transfer_b200 import _lib
     lib = _lib.load()
-    n, h, w, c, pad = 2, 8, 8, 64, 1
+    n, h, w = 2, 8, 8
     p = ctypes.c_void_p(1 << 20)
 
-    def img(dtype, hh=h, ww=w, sw=c):
+    def img(dtype, hh=h, ww=w, c=64, sw=None):
+        sw = sw or c
         return _lib.Image(1 << 20, dtype, n, hh, ww, c, hh * ww * sw, ww * sw, sw, 1)
     f32, bf16 = _lib.AST_F32, _lib.AST_BF16
-    for x, out, what in ((img(f32), img(bf16, h + 2, w + 2), b"dtype"),
-                         (img(bf16, sw=2 * c), img(bf16, h + 2, w + 2, sw=2 * c), b"dense")):
+    for x, pad, what in ((img(f32), 1, b"dtype"), (img(bf16, sw=128), 1, b"dense"),
+                         (img(bf16, c=24), 1, b"C=24 is not supported"), (img(bf16, c=1024), 4, b"cannot be staged")):
+        mixed, sw = what == b"dtype", x.sw if what == b"dense" else None
+        out = img(bf16 if mixed else x.dtype, h + 2 * pad, w + 2 * pad, x.c, sw)
         rc = lib.ast_instnorm_apply(ctypes.byref(x), p, p, p, p, None, ctypes.byref(out), pad, 1, None)
         assert rc < 0 and what in lib.ast_last_error(), lib.ast_last_error()
-        dx = img(out.dtype, sw=2 * c if what == b"dense" else c)
+        dx = img(out.dtype, c=x.c, sw=sw)
         rc = lib.ast_instnorm_bwd(ctypes.byref(x), p, p, p, p, ctypes.byref(out), pad, None, 1, p, p, p, ctypes.byref(dx),
                                   None, None)
         assert rc < 0 and what in lib.ast_last_error(), lib.ast_last_error()

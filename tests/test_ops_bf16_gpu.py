@@ -6,6 +6,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from test_instnorm_launch_kernels import check_bwd, probe_failures
+
 pytestmark = pytest.mark.gpu
 
 
@@ -37,14 +39,14 @@ def bf(x):
 
 def instnorm_bwd_reference(x, gamma, beta, gpad, pad, gextra, relu):
     """fp64 backward of ReflectionPad o ReLU o (+residual) o InstanceNorm on the device (CPU autograd at 10^8 elements is
-    too slow) -> fp32 mean / rstd, dbeta, dgamma, dx and g' (NHWC; g' only with gextra)."""
+    too slow) -> fp32 mean / rstd, dbeta, dgamma, dx and g' (NHWC; g' only with gextra; gpad may be None)."""
     xd = x.double().permute(0, 3, 1, 2).requires_grad_(True)
     gd, bd = gamma.double().requires_grad_(True), beta.double().requires_grad_(True)
     y = F.instance_norm(xd, weight=gd, bias=bd, eps=1e-5)
     if relu:
         y = F.relu(y)
     yp = F.pad(y, (pad,) * 4, mode="reflect") if pad else y
-    loss = (yp * gpad.double().permute(0, 3, 1, 2)).sum()
+    loss = (yp * gpad.double().permute(0, 3, 1, 2)).sum() if gpad is not None else 0
     if gextra is not None:
         loss = loss + (y * gextra.double().permute(0, 3, 1, 2)).sum()
     loss.backward()
@@ -53,8 +55,10 @@ def instnorm_bwd_reference(x, gamma, beta, gpad, pad, gextra, relu):
     gprime = None
     if gextra is not None:
         yr = F.instance_norm(xd.detach(), weight=gd.detach(), bias=bd.detach(), eps=1e-5)
-        gp = gpad.double().permute(0, 3, 1, 2)
-        fold = torch.autograd.functional.vjp(lambda t: F.pad(t, (pad,) * 4, mode="reflect") if pad else t, yr, gp)[1]
+        fold = 0
+        if gpad is not None:
+            gp = gpad.double().permute(0, 3, 1, 2)
+            fold = torch.autograd.functional.vjp(lambda t: F.pad(t, (pad,) * 4, mode="reflect") if pad else t, yr, gp)[1]
         gprime = ((fold + gextra.double().permute(0, 3, 1, 2)) * ((yr > 0) if relu else 1.0)).permute(0, 2, 3, 1)
     return mean, rstd, bd.grad, gd.grad, xd.grad.permute(0, 2, 3, 1), gprime
 
@@ -66,22 +70,45 @@ def instnorm_bwd_reference(x, gamma, beta, gpad, pad, gextra, relu):
     ("bf16", 2, 64, 64, 128, 0, True, False, 1), ("fp32", 2, 64, 64, 128, 1, True, False, 1),
     # production layers too large for L2: statistics, then apply
     ("bf16", 32, 128, 128, 64, 1, True, False, 2), ("bf16", 32, 256, 256, 32, 4, True, False, 2),
-    ("bf16", 16, 128, 128, 128, 1, False, True, 2), ("fp32", 32, 128, 128, 64, 1, True, False, 2)])
+    ("bf16", 16, 128, 128, 128, 1, False, True, 2), ("fp32", 32, 128, 128, 64, 1, True, False, 2),
+    # the staging plan's edges: a row of 257 pixels in two segments; three staged tensors (8 KB slabs) of 70 pixels in
+    # segments of 24, 24 and 22; pad 4 at h = w = 5 (every pixel folds mirrored positions)
+    ("bf16", 2, 9, 257, 32, 1, True, False, 1), ("bf16", 2, 16, 70, 128, 1, False, True, 1),
+    ("bf16", 2, 5, 5, 32, 4, True, False, 1), ("fp32", 2, 5, 5, 32, 4, False, True, 1),
+    # the channel counts at both ends of the consumer mapping (1 lane x 256 slots .. 128 lanes x 2 slots)
+    ("bf16", 2, 64, 64, 8, 1, True, False, 1), ("bf16", 2, 16, 16, 1024, 1, True, False, 1),
+    ("fp32", 2, 32, 32, 4, 1, True, False, 1), ("fp32", 2, 16, 16, 512, 1, True, False, 1),
+    # n = 1: one row per block; n = 300: one block per image, more blocks than fit at once -> two launches in L2
+    ("bf16", 1, 64, 64, 32, 1, True, False, 1), ("bf16", 300, 8, 8, 32, 1, True, False, 2),
+    # the L2 rule: x + g' of 103.7 MB and of 104.6 MB
+    ("bf16", 4, 225, 225, 128, 1, True, False, 1), ("bf16", 4, 226, 226, 128, 1, True, False, 2),
+    # only the skip gradient (no padded gradient)
+    ("bf16", 2, 64, 64, 128, 1, True, "only", 1),
+    # |mean| / std = 100 and 1000: sums of g' * xhat must stay within the conditioning of the maths (a sum of g' * x
+    # corrected by mean * sum g' afterwards does not: 2.3e-5 off in dgamma at 100, fp32, two launches).  fp32 without
+    # ReLU: at this ratio fp32 D = beta - A*mean moves the ReLU threshold by ~1e-5 std, which flips masks against the
+    # exact-mask norm pins below (check_bwd evaluates the mask as the kernel does)
+    ("bf16-mu100", 2, 64, 64, 128, 1, True, False, 1), ("fp32-mu100", 2, 64, 64, 128, 1, False, False, 1),
+    ("fp32-mu100", 16, 128, 128, 64, 1, False, True, 2), ("fp32-mu1000", 2, 64, 64, 128, 1, False, True, 1)])
 def test_instnorm_bwd_staged_bf16(env, dt, n, h, w, c, pad, relu, res, launches):
     """Backward of ReflectionPad o ReLU o (+residual) o InstanceNorm (cnn.py:58,68,91,98) against fp64 on the same rounded
     operands, on both sides of the library's size rule: the single cooperative kernel (second read from L2) and the
-    two launches give the same numbers."""
+    two launches give the same numbers.  res: the skip gradient gextra (and gtotal); "only": gextra without gpad.  A
+    "-muR" dtype draws x with |mean| / std = R.  Besides the norm-wise pins, every output is held element-wise to
+    the bounds of `check_bwd` (test_instnorm_launch_kernels.py), whose sum bounds scale with sum |g' * xhat|."""
     _lib, cg, ops = env
     torch.manual_seed(c + h + pad)
+    dt, _, mu = dt.partition("-")
     dtype = torch.bfloat16 if dt == "bf16" else torch.float32
-    x = (torch.randn(n, h, w, c, device="cuda") * 2 + 0.5).to(dtype)
+    x = ((torch.randn(n, h, w, c, device="cuda") * (2 / int(mu[2:])) + 2) if mu else
+         (torch.randn(n, h, w, c, device="cuda") * 2 + 0.5)).to(dtype)
     gamma = torch.rand(c, device="cuda") + 0.5
     beta = torch.randn(c, device="cuda") * 0.3
-    gpad = torch.randn(n, h + 2 * pad, w + 2 * pad, c, device="cuda").to(dtype)
+    gpad = torch.randn(n, h + 2 * pad, w + 2 * pad, c, device="cuda").to(dtype) if res != "only" else None
     gextra = torch.randn(n, h, w, c, device="cuda").to(dtype) if res else None
     mean, rstd, dbeta, dgamma, dx_ref, gprime = instnorm_bwd_reference(x, gamma, beta, gpad, pad, gextra, relu)
-    dx = torch.empty_like(x)
-    gtotal = torch.empty_like(x) if res else None
+    dx = torch.full_like(x, float("nan"))
+    gtotal = torch.full_like(x, float("nan")) if res else None
     s12 = torch.zeros(2, n * c, device="cuda")
     arrive = torch.zeros(n, dtype=torch.int32, device="cuda")
     before = _lib.family_stats()
@@ -89,8 +116,18 @@ def test_instnorm_bwd_staged_bf16(env, dt, n, h, w, c, pad, relu, res, launches)
     assert _lib.family_delta(before)["in_bwd"][0] == launches, f"{launches} InstanceNorm backward launch(es) expected"
     if launches == 1:
         assert int(arrive.min()) == int(arrive.max()) > 0
-    assert rel(s12[0].view(n, c).sum(0), dbeta) < 1e-5              # dbeta = sum g'
-    assert rel(s12[1].view(n, c).sum(0), dgamma) < 2e-5             # dgamma = sum g' xhat
+    rec = check_bwd(x, mean, rstd, gamma, beta, gpad, pad, gextra, relu, dx, gtotal, s12,
+                    torch.cuda.get_device_properties(0).multi_processor_count)
+    print(f"{(dt, mu, n, h, w, c, pad, relu, res)}: plan {rec['plan']}, k {rec['k']}: max err/bound dx "
+          f"{rec['ratio_dx']:.2e}, sums {rec['ratio_sums']:.2e}, all {rec['ratio']:.2e}; "
+          f"dgamma rel {rel(s12[1].view(n, c).sum(0), dgamma):.1e}; mutants {rec['mutants']}")
+    assert rec["plan"]["launches"] == launches
+    rec.update(entry="bwd", fams={}, want={}, inputs_changed=[], zero_on_entry=True,
+               arrive=(int(arrive.min()), int(arrive.max())))
+    assert not probe_failures(rec), probe_failures(rec)
+    if mu != "mu1000":   # there the fp32 rounding of the mean alone moves xhat by 6e-5 std against exact statistics
+        assert rel(s12[0].view(n, c).sum(0), dbeta) < 1e-5          # dbeta = sum g'
+        assert rel(s12[1].view(n, c).sum(0), dgamma) < 2e-5         # dgamma = sum g' xhat
     assert_bf16_close(dx, dx_ref, "dx")
     if res:        # gtotal = g' (the gradient handed to the residual skip)
         assert_bf16_close(gtotal, gprime, "gtotal")
